@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/sec of the OpenSora-v1.2 denoising loop on the vsb200 sm_100a path (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--pab]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--pab] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one iteration of the RFLOW sampling loop (schedulers/scheduling_rflow_open_sora.py:238-250 in the
@@ -18,6 +18,8 @@ other kernels), cpu_baseline (the oracle port on the host cores, bounded sample,
 the reference's eager path = the oracle restatement on torch/cuBLAS/SDPA library kernels on the same GPU), dsp_parity
 (N > 1: sharded == unsharded, bit for bit, before anything is timed), clocks, gpu_launches.
 --impl reference times the reference's CPU path (oracle port).
+--dump-outputs DIR writes the latents the last timed step returned (DIR/latent.npy from the resident arm, DIR/latent_e2e.npy
+from the host-buffer arm, float32): weights and inputs are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -217,6 +219,23 @@ def run_reference(args):
         "e2e": {"value": val, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes each tensor as <path>/<name>.npy in float32 (at most DUMP_LIMIT bytes in all); rank 0 only."""
+    import numpy as np
+
+    if int(os.environ.get("RANK", 0)) != 0:
+        return
+    size = sum(4 * t.numel() for t in arrays.values())
+    if size > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {size} bytes of outputs exceed {DUMP_LIMIT}")
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def _config(args, W):
@@ -458,6 +477,8 @@ def run_ours(args):
     # our launches inside the two timed regions: host launches + the launches baked into every replayed graph
     launches = ((kernels.launch_count() - l0) + (stepper.replayed_launches - r0)) // 2
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latent": state["z"], "latent_e2e": out_host})
 
     # ---- per-kernel pass: EAGER steps with CUDA-event pairs around every launch of ours (not part of value) ----
     eager = StepGraph(net, 7.0, enabled=False)
@@ -701,6 +722,8 @@ def run_cogvideox(args):
     net.reset_pab_state()
     sec_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs:  # the e2e arm leaves state["z"] alone; the profiled pass below advances it
+        dump_outputs(args.dump_outputs, {"latent": state["z"], "latent_e2e": out_host})
     net.reset_pab_state()
     kernels.PROFILE, kernels.PROFILE_KINDS = [], None
     sec_prof = timed(step_resident, args.steps)
@@ -798,6 +821,8 @@ def _simple_bench(args, name, net, one, n_sched, z_host, dt, frames, steps, conf
     net.reset_pab_state()
     sec_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs:  # the e2e arm leaves state["z"] alone; the profiled pass below advances it
+        dump_outputs(args.dump_outputs, {"latent": state["z"], "latent_e2e": out_host})
     net.reset_pab_state()
     kernels.PROFILE, kernels.PROFILE_KINDS = [], None
     sec_prof = timed(step_resident, args.steps)
@@ -965,7 +990,12 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from the host instead of replaying CUDA graphs")
     ap.add_argument("--first-step", type=int, default=-1, help="schedule index of the first timed step (default 0; 22 with --pab: inside the broadcast range)")
     ap.add_argument("--opt", action="append", default=[], help="kernel selection knob name=value (vsb_set_option)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the latents of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times a CPU sample, not the denoising step")
     if args.workload.startswith("cogvideox"):
         if args.impl == "reference":
             print(json.dumps({"impl": "reference", "unavailable": "the CPU reference arm is defined for the OpenSora workloads"}))

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- CPU/torch restatement of the CogVideoX transformer block (block level).
 
-PINNED against the reference's own CogVideoXTransformer3DModel, executed unmodified (tests/test_oracle_vs_reference.py::
+PINNED against the outputs of the reference's own CogVideoXTransformer3DModel, executed unmodified (tests/test_oracle_vs_reference.py::
 test_cogvideox_oracle_vs_reference_model: fp32 within summation order, bf16 and fp16 bit for bit; also
 test_cogvideox_layernorm_zero and the DDIM scheduler test).  ``diffusers==0.30.0`` (requirements.txt:25) is not installed
 here; oracle/ref_loader.load_cogvideox supplies the leaf classes the reference file imports from it:

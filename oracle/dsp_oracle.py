@@ -3,8 +3,8 @@
 The reference's comm layer cannot run on CPU (gloo has no list all_to_all; the gather asserts CUDA:
 core/distributed/comm.py:107,181), so the DSP oracle is the invariant the reference relies on:
 every per-rank tensor is a slice of the zero-padded full tensor (SURVEY.md Appendix E).  Pinned in
-tests/test_oracle_vs_reference.py by running the reference's own functions on simulated ranks
-(threads + a fake ``dist``).
+tests/test_oracle_vs_reference.py against the outputs of the reference's own functions run on simulated ranks
+(threads + a fake ``dist``, oracle/gen_golden_pins.py).
 """
 from typing import List
 

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- CPU/torch restatement of the Latte transformer blocks (block level).
 
-PINNED against the reference's own LatteT2V, executed unmodified (tests/test_oracle_vs_reference.py::
+PINNED against the outputs of the reference's own LatteT2V, executed unmodified (tests/test_oracle_vs_reference.py::
 test_latte_oracle_vs_reference_model: fp32 within summation order, bf16 bit for bit).  ``diffusers==0.30.0`` (requirements.txt:25)
 is not installed here, so the reference file's diffusers LEAF classes are supplied by oracle/ref_loader.load_latte from the
 reference's own vendored copies in open_sora_plan_v110_transformer_3d.py (Attention + AttnProcessor2_0, PatchEmbed,

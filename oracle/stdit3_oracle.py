@@ -7,8 +7,8 @@ package (``videosys_b200``); only ``tests/``, ``__graft_entry__.smoke()`` and ``
 Every function is a functional restatement (state_dict in, tensors out; no nn.Module, no global
 singletons) of the reference code it cites, keeping the reference's *op order and rounding points*:
 each eager op rounds to the storage dtype exactly where the reference's eager op does, so on CPU in
-the same dtype the two are bit-identical (pinned in tests/test_oracle_vs_reference.py, which runs
-wherever ``/root/reference`` exists, and by the committed golden vectors in tests/golden/).
+the same dtype the two are bit-identical (pinned by the committed golden vectors in tests/golden/, which
+tests/test_oracle_vs_reference.py and tests/test_oracle_golden.py check).
 
 Third-party pieces that are not in the reference tree and are restated from their published
 semantics (SURVEY.md section 8c): timm ``Mlp`` (fc2(act(fc1(x)))), ``rotary_embedding_torch``

@@ -39,6 +39,11 @@ def normalish(name: str, shape, std=1.0) -> torch.Tensor:
     return acc * (std * (3.0 / 4.0) ** 0.5)
 
 
+def copied(k: str, v: torch.Tensor) -> bool:
+    """The entries fill_state_dict keeps as they are: integer buffers and rotary frequency tables."""
+    return not torch.is_floating_point(v) or k.endswith("rope.freqs") or k.endswith("inv_freq")
+
+
 def fill_state_dict(sd: dict, tag: str, weight_std: float = 0.05) -> dict:
     """Deterministic weights for every floating tensor of a STDiT3-style state_dict (keeps dtypes).
 
@@ -48,10 +53,7 @@ def fill_state_dict(sd: dict, tag: str, weight_std: float = 0.05) -> dict:
     """
     out = {}
     for k, v in sd.items():
-        if not torch.is_floating_point(v):
-            out[k] = v.clone()
-            continue
-        if k.endswith("rope.freqs") or k.endswith("inv_freq"):
+        if copied(k, v):
             out[k] = v.clone()
             continue
         if k.endswith("q_norm.weight") or k.endswith("k_norm.weight"):

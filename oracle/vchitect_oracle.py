@@ -4,8 +4,8 @@ Follows models/transformers/vchitect_transformer_3d.py (JointTransformerBlock.fo
 and models/modules/attentions.py (VchitectAttnProcessor :641-949: apply_rotary_emb :688-701, spatial_attn :663-705,
 temporal_attention :707-768, cross_attention :770-803, __call__ :805-927), sp_size == 1, PAB via the callback gates.
 
-Pinning (tests/test_oracle_vs_reference.py): ``attention`` (the whole processor on a VchitectAttention's parameters) bit for
-bit against the reference's own VchitectAttention + VchitectAttnProcessor, incl. the PAB gates
+Pinning (tests/test_oracle_vs_reference.py, against stored outputs of the reference): ``attention`` (the whole processor on a
+VchitectAttention's parameters) bit for bit against the reference's own VchitectAttention + VchitectAttnProcessor, incl. the PAB gates
 (test_vchitect_attention_vs_reference, test_vchitect_attention_pab_vs_reference); ``transformer_forward`` against the
 reference's VchitectXLTransformerModel executed unmodified (test_vchitect_oracle_vs_reference_model: fp32 within summation
 order, bf16 bit for bit).  diffusers==0.30.0 is not installed here: for that run oracle/ref_loader.load_vchitect supplies the

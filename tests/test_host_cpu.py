@@ -163,7 +163,8 @@ def _dsp_worker(rank, world, port, T, S, q):
 
 
 @pytest.mark.parametrize("T,S", [(5, 9), (4, 8)])
-def test_dsp_comm_gloo_world2(T, S):
+def test_dsp_comm_gloo_world2(monkeypatch, T, S):
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")  # CPU ranks on gloo: with a GPU visible, initialize() picks NCCL
     world, port = 2, 29600 + (os.getpid() % 200) + T
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
@@ -212,9 +213,10 @@ def _ulysses_worker(rank, world, port, q):
         q.put((rank, None, None, traceback.format_exc()))
 
 
-def test_ulysses_head_scatter_gloo_world2():
+def test_ulysses_head_scatter_gloo_world2(monkeypatch):
     """CogVideoX's head-scatter exchange (reference cogvideox_transformer_3d.py:44-165): after the scatter a rank holds
     every row of its head group, after the way back its own rows (text + its chunk) with every head."""
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")  # CPU ranks on gloo: with a GPU visible, initialize() picks NCCL
     world, port = 2, 29800 + (os.getpid() % 150)
     ctx = mp.get_context("spawn")
     q = ctx.Queue()

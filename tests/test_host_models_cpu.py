@@ -248,13 +248,14 @@ def _sp_worker(rank, world, port, which, enable_cp, q):
 @pytest.mark.parametrize("which,enable_cp", [("osp_v110", False), ("osp_v110", True), ("latte", False), ("cogvideox", False),
                                              ("cogvideox", True), ("osp_v120", False), ("stdit3", False),
                                              ("cogvideox_rope", False)])
-def test_model_parallelism_gloo_world2(which, enable_cp):
+def test_model_parallelism_gloo_world2(monkeypatch, which, enable_cp):
     """Two ranks: frame-sharded DSP (Latte / Open-Sora-Plan v1.1.0: temporal blocks switch to a patch shard, with the RoPE
     tables following the switch), head-scatter sequence parallelism (CogVideoX) or CFG parallelism reproduce the single-rank
     forward on every rank (fp32; the exchanges move data, the per-sequence arithmetic is unchanged)."""
     import multiprocessing as mp
     import os
 
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")  # CPU ranks on gloo: with a GPU visible, initialize() picks NCCL
     world, port = 2, 30100 + (os.getpid() % 300) + 7 * ["osp_v110", "latte", "cogvideox", "osp_v120", "stdit3", "cogvideox_rope"].index(which) + int(enable_cp)
     ctx = mp.get_context("spawn")
     q = ctx.Queue()

@@ -1,378 +1,237 @@
-"""Pins the oracle by EXECUTING THE UNMODIFIED REFERENCE (only where /root/reference exists: the
-authoring container).  On the GPU box these skip; the golden vectors carry the pin there."""
-import threading
+"""Pins the oracle and the product's host logic to outputs of the UNMODIFIED reference.
+
+tests/golden/reference_pins.pt.gz holds, for every check below, what the reference computed on the same synthetic weights and
+inputs (oracle/gen_golden_pins.py executes it, with the configurations and input helpers of this module), in the compact
+records of oracle/pins.py: bit-exact comparisons as SHA-256 digests, tolerance comparisons as a fixed sample plus whole-
+tensor sums.  The weights are regenerated here from the reference's state-dict templates stored alongside."""
+import os
 
 import pytest
 import torch
 
-from oracle import cases, dsp_oracle, pab_oracle, ref_loader, stdit3_oracle as O, synth
+from oracle import cases, dsp_oracle, pab_oracle, pin_cases as PC, pins, stdit3_oracle as O, synth
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not mounted")
+
+
+@pytest.fixture(scope="module")
+def pin(golden_dir):
+    return pins.load(os.path.join(golden_dir, "reference_pins.pt.gz"))
+
+
+def _fill(pin, key, tag):
+    return pins.filled(pin["tmpl." + key], tag)
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_forward_bit_exact(dtype):
+def test_forward_bit_exact(pin, dtype):
     c = cases.small_model_cfg(depth=2)
-    net = ref_loader.build_stdit3(dtype=dtype, **c)
-    sd = synth.fill_state_dict(net.state_dict(), "vsref.")
-    net.load_state_dict(sd)
+    sd = _fill(pin, f"stdit3.{PC.DT[dtype]}", "vsref.")
     inp = cases.forward_inputs(dtype)
     with torch.no_grad():
-        ref = net(inp["x"], inp["timestep"], inp["y"], mask=inp["mask"], x_mask=inp["x_mask"], fps=inp["fps"],
-                  height=inp["height"], width=inp["width"])
         out = O.stdit3_forward(sd, cases.oracle_cfg(c), **inp)
-    assert torch.equal(ref, out)
+    pins.assert_exact(out, pin[f"stdit3.forward.{PC.DT[dtype]}"])
 
 
-def test_forward_with_pab_bit_exact_over_steps():
+def test_forward_with_pab_bit_exact_over_steps(pin):
     """PAB on (attn + cross broadcast; mlp_broadcast=False, the only mode the reference can run for
     OpenSora, SURVEY fact 7): reuse-by-reference semantics and counters over 8 consecutive steps."""
-    ref = ref_loader.load()
-    P = ref.pab_mgr
     dtype = torch.bfloat16
     c = cases.small_model_cfg(depth=2)
-    net = ref_loader.build_stdit3(dtype=dtype, **c)
-    sd = synth.fill_state_dict(net.state_dict(), "vsref.")
-    net.load_state_dict(sd)
-    steps = [1000, 900, 860, 800, 700, 600, 500, 300]
-    P.set_pab_manager(P.PABConfig(spatial_broadcast=True, spatial_threshold=[450, 930], spatial_range=2,
-                                  temporal_broadcast=True, temporal_threshold=[450, 930], temporal_range=4,
-                                  cross_broadcast=True, cross_threshold=[450, 930], cross_range=6))
-    P.update_steps(len(steps))
+    sd = _fill(pin, "stdit3.bfloat16", "vsref.")
+    steps = PC.OPENSORA_PAB_STEPS
     gate = pab_oracle.opensora_default(len(steps))
     states = {k: [O.BlockPABState() for _ in range(2)] for k in ("spatial", "temporal")}
     inp = cases.forward_inputs(dtype)
-    try:
-        with torch.no_grad():
-            for i, t in enumerate(steps):
-                inp["x"] = synth.normalish(f"pab.x{i}", tuple(inp["x"].shape))
-                inp["timestep"] = torch.tensor([float(t)] * 2)
-                r = net(inp["x"], inp["timestep"], inp["y"], mask=inp["mask"], x_mask=inp["x_mask"], fps=inp["fps"],
-                        height=inp["height"], width=inp["width"])
-                o = O.stdit3_forward(sd, cases.oracle_cfg(c), pab=gate, pab_states=states, **inp)
-                assert torch.equal(r, o), f"step {i} t={t}"
-    finally:
-        P.PAB_MANAGER = None
+    with torch.no_grad():
+        for i, t in enumerate(steps):
+            inp["x"] = synth.normalish(f"pab.x{i}", tuple(inp["x"].shape))
+            inp["timestep"] = torch.tensor([float(t)] * 2)
+            o = O.stdit3_forward(sd, cases.oracle_cfg(c), pab=gate, pab_states=states, **inp)
+            pins.assert_exact(o, pin[f"stdit3.pab.{i}"], f"step {i} t={t}")
 
 
-def test_pab_gate_matches_reference_manager():
-    P = ref_loader.load().pab_mgr
-    import random
-
-    rnd = random.Random(0)
-    try:
-        for _ in range(20):
-            kw = {}
-            spec = {}
-            for k in ("spatial", "temporal", "cross"):
-                on = rnd.random() < 0.7
-                lo = rnd.randrange(0, 600)
-                hi = lo + rnd.randrange(1, 500)
-                rg = rnd.randrange(1, 7)
-                kw.update({f"{k}_broadcast": on, f"{k}_threshold": [lo, hi], f"{k}_range": rg})
-                spec[k] = (on, (lo, hi), rg)
-            steps = rnd.randrange(1, 40)
-            P.set_pab_manager(P.PABConfig(**kw))
-            P.update_steps(steps)
-            g = pab_oracle.PABGate(steps=steps, **spec)
-            for k, fn in (("spatial", P.if_broadcast_spatial), ("temporal", P.if_broadcast_temporal), ("cross", P.if_broadcast_cross)):
-                c1 = c2 = 0
-                for _ in range(3 * steps):
-                    t = rnd.choice([None, rnd.randrange(0, 1100)])
-                    f1, c1 = fn(t, c1)
-                    f2, c2 = g.gate(k, t, c2)
-                    assert (f1, c1) == (f2, c2)
-    finally:
-        P.PAB_MANAGER = None
+def test_pab_gate_matches_reference_manager(pin):
+    got = []
+    for spec, steps, ts in PC.pab_gate_cases():
+        g = pab_oracle.PABGate(steps=steps, **spec)
+        for k in ("spatial", "temporal", "cross"):
+            c2 = 0
+            for t in ts[k]:
+                f2, c2 = g.gate(k, t, c2)
+                got.append((int(f2), c2))
+    pins.assert_exact(torch.tensor(got, dtype=torch.int64), pin["pab_gate"], "(broadcast, counter) after every call")
 
 
-class _FakeDist:
-    """Thread-per-rank stand-in for torch.distributed so the reference comm functions run on CPU."""
-
-    def __init__(self, sp):
-        self.sp = sp
-        self.board = [None] * sp
-        self.bar = threading.Barrier(sp)
-        self.local = threading.local()
-        self.ProcessGroup = object
-
-    def get_world_size(self, group=None):
-        return self.sp
-
-    def get_rank(self, group=None):
-        return self.local.rank
-
-    def all_to_all(self, output_list, input_list, group=None):
-        r = self.local.rank
-        self.board[r] = input_list
-        self.bar.wait()
-        for src in range(self.sp):
-            output_list[src].copy_(self.board[src][r])
-        self.bar.wait()
-
-
-def _run_ranks(sp, fn):
-    fake = _FakeDist(sp)
-    comm = ref_loader.load().comm
-    old = comm.dist
-    comm.dist = fake
-    outs, errs = [None] * sp, []
-
-    def body(r):
-        fake.local.rank = r
-        try:
-            outs[r] = fn(comm, r)
-        except Exception as e:  # pragma: no cover
-            errs.append(e)
-            fake.bar.abort()
-
-    try:
-        th = [threading.Thread(target=body, args=(r,)) for r in range(sp)]
-        [t.start() for t in th]
-        [t.join() for t in th]
-    finally:
-        comm.dist = old
-    assert not errs, errs
-    return outs
-
-
-@pytest.mark.parametrize("sp,T,S", [(2, 5, 9), (4, 5, 9), (8, 20, 24), (4, 4, 8), (2, 15, 405)])
-def test_dsp_reshard_matches_reference_comm(sp, T, S):
+@pytest.mark.parametrize("sp,T,S", PC.DSP_CASES)
+def test_dsp_reshard_matches_reference_comm(pin, sp, T, S):
     B, C = 2, 16
     full = synth.normalish(f"dsp{sp}{T}{S}", (B, T, S, C))
     tp, spd = dsp_oracle.pad_amount(T, sp), dsp_oracle.pad_amount(S, sp)
     res = dsp_oracle.split_sequence(full, sp, dim=2)
-
-    def fn(comm, r):
-        x = comm._split_sequence_func(full, None, 2, spd)
-        a = comm.all_to_all_with_pad(x, None, scatter_dim=1, gather_dim=2, scatter_pad=tp, gather_pad=spd)
-        b = comm.all_to_all_with_pad(a, None, scatter_dim=2, gather_dim=1, scatter_pad=spd, gather_pad=tp)
-        return x, a, b
-
-    outs = _run_ranks(sp, fn)
     parts = [p.reshape(B, -1, C) for p in res]
     sw, new_s, new_t = dsp_oracle.dynamic_switch(parts, T, S, to_spatial_shard=False)
     back, s2, t2 = dsp_oracle.dynamic_switch(sw, T, S, to_spatial_shard=True)
     padded_t = torch.cat([full, torch.zeros(B, tp, S, C)], 1)
+    recs = pin[f"dsp.{sp}.{T}.{S}"]
+    assert len(recs) == sp
     for r in range(sp):
-        x, a, b = outs[r]
-        assert torch.equal(x, res[r])
-        assert torch.equal(a.reshape(B, -1, C), sw[r]) and (a.shape[1], a.shape[2]) == (new_t, new_s)
-        assert torch.equal(a, padded_t[:, r * new_t:(r + 1) * new_t])  # Appendix E: a slice of the T-padded tensor
-        assert torch.equal(b.reshape(B, -1, C), back[r]) and torch.equal(b, x)
-    assert torch.equal(dsp_oracle.gather_sequence([o[2] for o in outs], 2, spd), full)
+        rx, ra, rb = recs[r]
+        pins.assert_exact(res[r], rx, f"rank {r} split")
+        a = padded_t[:, r * new_t:(r + 1) * new_t]  # Appendix E: a slice of the T-padded tensor
+        pins.assert_exact(a, ra, f"rank {r} to temporal shard")
+        assert ra["shape"][1:3] == (new_t, new_s) and torch.equal(a.reshape(B, -1, C), sw[r])
+        pins.assert_exact(back[r].reshape(res[r].shape), rb, f"rank {r} back to spatial shard")
+        assert rb == rx
+    assert torch.equal(dsp_oracle.gather_sequence(res, 2, spd), full)
+
+
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_cogvideox_layernorm_zero(dtype):
+def test_cogvideox_layernorm_zero(pin, dtype):
     """The in-tree half of the CogVideoX block: CogVideoXLayerNormZero (models/modules/normalization.py:36-57)."""
     from oracle import cogvideox_oracle as CO
 
-    N = ref_loader.load().normalization
-    mod = N.CogVideoXLayerNormZero(64, 128, True, 1e-5, bias=True).to(dtype)
-    sd = {"n." + k: v for k, v in synth.fill_state_dict(mod.state_dict(), "lnz.").items()}
+    sd = {"n." + k: v for k, v in _fill(pin, f"lnz.{PC.DT[dtype]}", "lnz.").items()}
     sd["n.norm.weight"] = (1 + 0.2 * synth.uniform("lnz.w", (128,))).to(dtype)
-    mod.load_state_dict({k[2:]: v for k, v in sd.items()})
-    h = synth.normalish("lnz.h", (2, 9, 128)).to(dtype)
-    e = synth.normalish("lnz.e", (2, 4, 128)).to(dtype)
-    t = synth.normalish("lnz.t", (2, 64)).to(dtype)
     with torch.no_grad():
-        ref = mod(h, e, t)
-        got = CO.layer_norm_zero(sd, "n.", h, e, t)
-    for a, b in zip(ref, got):
-        assert torch.equal(a, b)
+        got = CO.layer_norm_zero(sd, "n.", *PC.lnz_inputs(dtype))
+    want = pin[f"lnz.{PC.DT[dtype]}"]
+    assert len(got) == len(want)
+    for a, rec in zip(got, want):
+        pins.assert_exact(a, rec)
 
 
-def test_cogvideox_ddim_scheduler_vs_reference():
-    """videosys_b200's CogVideoXDDIMScheduler against the reference's own class (executed unmodified): trailing timesteps,
-    the SNR-shifted / zero-terminal-SNR alphas, and 50 v-prediction steps on random tensors."""
-    if not ref_loader.available():
-        pytest.skip("reference tree not present")
+
+
+def test_cogvideox_ddim_scheduler_vs_reference(pin):
+    """videosys_b200's CogVideoXDDIMScheduler against the reference's own class: trailing timesteps, the SNR-shifted /
+    zero-terminal-SNR alphas, and 50 v-prediction steps on random tensors."""
     from videosys_b200.schedulers.scheduling_ddim_cogvideox import CogVideoXDDIMScheduler as Ours
 
-    Ref = ref_loader.load_cogvideox_scheduler()
-    kw = dict(num_train_timesteps=1000, beta_start=0.00085, beta_end=0.012, beta_schedule="scaled_linear", clip_sample=False,
-              set_alpha_to_one=True, steps_offset=0, prediction_type="v_prediction", timestep_spacing="trailing",
-              rescale_betas_zero_snr=True, snr_shift_scale=3.0)
-    ref, ours = Ref(**kw), Ours(**kw)
-    assert torch.equal(ref.alphas_cumprod, ours.alphas_cumprod)
+    rec = pin["cogx_ddim"]
+    ours = Ours(**PC.COGX_DDIM)
+    pins.assert_exact(ours.alphas_cumprod, rec["alphas_cumprod"])
     for n in (50, 30, 7):
-        ref.set_timesteps(n)
         ours.set_timesteps(n)
-        assert ref.timesteps.tolist() == ours.timesteps.tolist()
-    ref.set_timesteps(50)
+        assert ours.timesteps.tolist() == rec["timesteps"][n]
     ours.set_timesteps(50)
     g = torch.Generator().manual_seed(0)
-    x = torch.randn(1, 3, 4, 6, 6, generator=g)
-    xr, xo = x.clone(), x.clone()
-    for t in ref.timesteps:
-        v = torch.randn(x.shape, generator=g)
-        xr = ref.step(v, t, xr, return_dict=False)[0]
+    xo = torch.randn(1, 3, 4, 6, 6, generator=g)
+    assert len(rec["steps"]) == len(ours.timesteps)
+    for t, want in zip(rec["timesteps"][50], rec["steps"]):
+        v = torch.randn(xo.shape, generator=g)
         xo = ours.step(v, int(t), xo)[0]
-        assert torch.allclose(xr.float(), xo.float(), rtol=1e-5, atol=1e-6), int(t)
-
-
-def _vchitect_ref_attention(C, H, context_pre_only, dtype):
-    A = ref_loader.load().attentions
-    attn = A.VchitectAttention(query_dim=C, cross_attention_dim=None, added_kv_proj_dim=C, dim_head=C // H, heads=H,
-                               out_dim=C, context_pre_only=context_pre_only, bias=True, processor=A.VchitectAttnProcessor())
-    attn = attn.to(dtype).eval()
-    attn.parallel_manager = ref_loader.SingleRankPM()
-    sd = synth.fill_state_dict(attn.state_dict(), "vchattn.")
-    attn.load_state_dict(sd)
-    return attn, {"a." + k: v for k, v in sd.items()}
+        pins.assert_close(xo.float(), want, rtol=1e-5, atol=1e-6, what=int(t))
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-@pytest.mark.parametrize("Fr,S,L,pre_only", [(5, 12, 7, False), (5, 12, 7, True), (1, 12, 7, False)])
-def test_vchitect_attention_vs_reference(Fr, S, L, pre_only, dtype):
+@pytest.mark.parametrize("Fr,S,L,pre_only", PC.VCH_ATTN_CASES)
+def test_vchitect_attention_vs_reference(pin, Fr, S, L, pre_only, dtype):
     """oracle/vchitect_oracle.attention against the reference's own VchitectAttention + VchitectAttnProcessor
-    (models/modules/attentions.py:321-949, executed unmodified): temporal (RoPE), cross (frame-0 text keys) and spatial
-    joint attention, the 1.1 mix, the output projections of both streams; bit for bit."""
+    (models/modules/attentions.py:321-949): temporal (RoPE), cross (frame-0 text keys) and spatial joint attention, the
+    1.1 mix, the output projections of both streams; bit for bit."""
     from oracle import vchitect_oracle as VO
 
-    C, H = 64, 4
-    attn, sd = _vchitect_ref_attention(C, H, pre_only, dtype)
+    C, H = PC.VCH_ATTN_C, PC.VCH_ATTN_H
+    sd = {"a." + k: v for k, v in _fill(pin, f"vch_attn.{int(pre_only)}.{PC.DT[dtype]}", "vchattn.").items()}
     nh = synth.normalish("vch.h", (Fr, S, C)).to(dtype)
     ne = synth.normalish("vch.e", (Fr, L, C)).to(dtype)
     fc = VO.freqs_cis(C // H, 64, theta=1e6)
     with torch.no_grad():
-        rv, re = attn(hidden_states=nh, encoder_hidden_states=ne, freqs_cis=fc, full_seqlen=Fr, Frame=Fr,
-                      timestep=torch.tensor([500]))
         ov, oe = VO.attention(sd, "a.", nh, ne, fc, H, Fr, pre_only)
-    assert torch.equal(rv, ov)
-    assert torch.equal(re, oe)
+    rv, re = pin[f"vch_attn.{Fr}.{S}.{L}.{int(pre_only)}.{PC.DT[dtype]}"]
+    pins.assert_exact(ov, rv, "video stream")
+    pins.assert_exact(oe, re, "text stream")
 
 
-def test_vchitect_attention_pab_vs_reference():
+def test_vchitect_attention_pab_vs_reference(pin):
     """The three PAB gates of the processor (:838-895: temporal, cross, spatial, in this order) over 8 steps."""
     from oracle import vchitect_oracle as VO
 
-    ref = ref_loader.load()
-    P = ref.pab_mgr
-    C, H, Fr, S, L = 64, 4, 4, 10, 6
-    attn, sd = _vchitect_ref_attention(C, H, False, torch.float32)
-    cfg = P.PABConfig(spatial_broadcast=True, spatial_threshold=[100, 800], spatial_range=2, temporal_broadcast=True,
-                      temporal_threshold=[100, 800], temporal_range=3, cross_broadcast=True, cross_threshold=[100, 800],
-                      cross_range=4)
-    P.set_pab_manager(cfg)
-    P.update_steps(8)
-    try:
-        fc = VO.freqs_cis(C // H, 64, theta=1e6)
-        counts = {"spatial": 0, "temporal": 0, "cross": 0}
-        cache = {}
-        G = pab_oracle.PABGate((True, (100, 800), 2), (True, (100, 800), 3), (True, (100, 800), 4), 8)
-        for step, t in enumerate([900, 700, 650, 600, 550, 500, 450, 50]):
-            nh = synth.normalish(f"vchp.h{step}", (Fr, S, C))
-            ne = synth.normalish(f"vchp.e{step}", (Fr, L, C))
+    (C, H), (Fr, S, L) = (PC.VCH_ATTN_C, PC.VCH_ATTN_H), PC.VCH_ATTN_PAB_SHAPE
+    sd = {"a." + k: v for k, v in _fill(pin, "vch_attn.0.float32", "vchattn.").items()}
+    fc = VO.freqs_cis(C // H, 64, theta=1e6)
+    counts = {"spatial": 0, "temporal": 0, "cross": 0}
+    cache = {}
+    G = PC.pab_gate(PC.VCH_ATTN_PAB_KW, len(PC.PAB_TS))
+    for step, t in enumerate(PC.PAB_TS):
+        nh = synth.normalish(f"vchp.h{step}", (Fr, S, C))
+        ne = synth.normalish(f"vchp.e{step}", (Fr, L, C))
 
-            def gate(kind, t=t):
-                hit, counts[kind] = G.gate(kind, t, counts[kind])
-                return hit
+        def gate(kind, t=t):
+            hit, counts[kind] = G.gate(kind, t, counts[kind])
+            return hit
 
-            with torch.no_grad():
-                rv, re = attn(hidden_states=nh, encoder_hidden_states=ne, freqs_cis=fc, full_seqlen=Fr, Frame=Fr,
-                              timestep=torch.tensor([t]))
-                ov, oe = VO.attention(sd, "a.", nh, ne, fc, H, Fr, False, gate, cache)
-            assert torch.equal(rv, ov) and torch.equal(re, oe), step
-    finally:
-        P.PAB_MANAGER = None
+        with torch.no_grad():
+            ov, oe = VO.attention(sd, "a.", nh, ne, fc, H, Fr, False, gate, cache)
+        rv, re = pin[f"vch_attn_pab.{step}"]
+        pins.assert_exact(ov, rv, step)
+        pins.assert_exact(oe, re, step)
 
 
 # ---- Open-Sora-Plan v1.1.0: the product's host logic against the UNMODIFIED reference model --------------------------------
-OSP_SMALL = dict(num_attention_heads=2, attention_head_dim=72, in_channels=4, out_channels=8, num_layers=2,
-                 cross_attention_dim=144, attention_bias=True, sample_size=(8, 8), patch_size=2, activation_fn="gelu-approximate",
-                 norm_type="ada_norm_single", norm_elementwise_affine=False, norm_eps=1e-6, caption_channels=32, video_length=5,
-                 attention_mode="math", use_rope=True)
 
 
-def _osp_pair(cfg, tag="osp."):
+
+
+def _osp_net(pin, cfg, key, tag):
     from videosys_b200.models.transformers.open_sora_plan_v110_transformer_3d import LatteT2V
 
-    ref = ref_loader.build_osp_v110(**cfg)
-    sd = synth.fill_state_dict(ref.state_dict(), tag)
-    ref.load_state_dict(sd)
     net = LatteT2V(**cfg)
-    net.load_state_dict(sd)  # strict: same parameter / buffer names as the reference
-    return ref, net.eval()
+    net.load_state_dict(_fill(pin, key, tag))  # strict: same parameter / buffer names as the reference
+    return net.eval()
 
 
-def _osp_inputs(B, Fr, HW, L=7, tag="osp."):
-    x = synth.normalish(tag + "x", (B, 4, Fr, *HW))
-    enc = synth.normalish(tag + "enc", (B, 1, L, 32))
-    m = torch.ones(B, 1, L)
-    m[B - 1, 0, L - 2:] = 0  # tokenizer padding on the last sample
-    return x, enc, m
 
 
-@pytest.mark.parametrize("use_rope,HW,scale1d", [(True, (8, 8), None), (False, (8, 8), None), (True, (12, 8), 2)])
-def test_osp_v110_mirror_vs_reference_model(monkeypatch, use_rope, HW, scale1d):
+@pytest.mark.parametrize("use_rope,HW,scale1d", PC.OSP_MIRROR_CASES)
+def test_osp_v110_mirror_vs_reference_model(pin, monkeypatch, use_rope, HW, scale1d):
     """videosys_b200's Open-Sora-Plan v1.1.0 front end, its kernel entries replaced by torch stand-ins
-    (tests/kernels_emul.py), against the reference's own LatteT2V executed unmodified (oracle/ref_loader.load_osp_v110):
-    RoPE tables (2-D / 1-D, linear scaling), position tables, text padding mask, block order, output head."""
+    (tests/kernels_emul.py), against the reference's own LatteT2V: RoPE tables (2-D / 1-D, linear scaling), position tables,
+    text padding mask, block order, output head."""
     from tests import kernels_emul
 
     kernels_emul.emulate(monkeypatch)
-    ref, net = _osp_pair(dict(OSP_SMALL, use_rope=use_rope, interpolation_scale_1d=scale1d))
+    key = PC.osp_key(use_rope, HW, scale1d)
+    net = _osp_net(pin, dict(PC.OSP_SMALL, use_rope=use_rope, interpolation_scale_1d=scale1d), key, "osp.")
     B, Fr = 2, 5
-    x, enc, m = _osp_inputs(B, Fr, HW)
-    t = torch.tensor([500, 500])
-    with torch.no_grad():
-        want = ref(x, timestep=t, all_timesteps=torch.tensor([900, 500]), encoder_hidden_states=enc,
-                   added_cond_kwargs={"resolution": None, "aspect_ratio": None}, attention_mask=torch.ones(B, Fr, *HW),
-                   encoder_attention_mask=m, return_dict=False)[0]
-    got = net(x, timestep=t, all_timesteps=[900, 500], encoder_hidden_states=enc, attention_mask=torch.ones(B, Fr, *HW),
-              encoder_attention_mask=m, return_dict=False)[0]
-    assert got.shape == want.shape
-    assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
+    x, enc, m = PC.osp_inputs(B, Fr, HW)
+    got = net(x, timestep=torch.tensor([500, 500]), all_timesteps=[900, 500], encoder_hidden_states=enc,
+              attention_mask=torch.ones(B, Fr, *HW), encoder_attention_mask=m, return_dict=False)[0]
+    pins.assert_close(got, pin[key], rtol=1e-4, atol=1e-5)
 
 
-def test_osp_v110_pab_vs_reference_model(monkeypatch):
+def test_osp_v110_pab_vs_reference_model(pin, monkeypatch):
     """Eight steps with PAB (attention broadcast on all three gates + the MLP skip windows) on both sides."""
     from tests import kernels_emul
     from videosys_b200.core.pab import pab_mgr as ours
 
     kernels_emul.emulate(monkeypatch)
-    P = ref_loader.load().pab_mgr
-    ref, net = _osp_pair(OSP_SMALL, "ospp.")
-    ts = [900, 700, 650, 600, 550, 500, 450, 50]
-    mlp = {700: {"block": [0, 1], "skip_count": 2}, 550: {"block": [1], "skip_count": 1}}
-    kw = dict(spatial_broadcast=True, spatial_threshold=[100, 850], spatial_range=2, temporal_broadcast=True,
-              temporal_threshold=[100, 850], temporal_range=3, cross_broadcast=True, cross_threshold=[100, 850], cross_range=4,
-              mlp_broadcast=True, mlp_spatial_broadcast_config=mlp, mlp_temporal_broadcast_config=mlp)
-    P.set_pab_manager(P.PABConfig(**kw))
-    P.update_steps(len(ts))
-    ours.set_pab_manager(ours.PABConfig(**kw))
-    ours.update_steps(len(ts))
+    net = _osp_net(pin, PC.OSP_SMALL, "ospp", "ospp.")
+    ours.set_pab_manager(ours.PABConfig(**PC.OSP_PAB_KW))
+    ours.update_steps(len(PC.PAB_TS))
     net.reset_pab_state()
     try:
         B, Fr, HW = 2, 5, (8, 8)
-        for step, t in enumerate(ts):
-            x, enc, m = _osp_inputs(B, Fr, HW, tag=f"ospp{step}.")
-            tt = torch.tensor([t, t])
-            with torch.no_grad():
-                want = ref(x, timestep=tt, all_timesteps=torch.tensor(ts), encoder_hidden_states=enc,
-                           added_cond_kwargs={"resolution": None, "aspect_ratio": None}, attention_mask=torch.ones(B, Fr, *HW),
-                           encoder_attention_mask=m, return_dict=False)[0]
-            got = net(x, timestep=tt, all_timesteps=ts, encoder_hidden_states=enc, encoder_attention_mask=m,
+        for step, t in enumerate(PC.PAB_TS):
+            x, enc, m = PC.osp_inputs(B, Fr, HW, tag=f"ospp{step}.")
+            got = net(x, timestep=torch.tensor([t, t]), all_timesteps=PC.PAB_TS, encoder_hidden_states=enc, encoder_attention_mask=m,
                       return_dict=False)[0]
-            assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (step, (got - want).abs().max())
+            pins.assert_close(got, pin[f"ospp.{step}"], rtol=1e-4, atol=1e-5, what=step)
     finally:
-        P.PAB_MANAGER = None
         ours.set_pab_manager(None)
 
 
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16, torch.float32])
-def test_osp_v110_rope_tables_vs_reference_classes(dtype):
+def test_osp_v110_rope_tables_vs_reference_classes(pin, dtype):
     """The cos / signed-sin tables of vsb_qk_rope_halves against LinearScalingRoPE2D / LinearScalingRoPE1D run on q itself:
     q*cos + partner*sin_signed, evaluated op by op in the dtype, equals the reference's output bit for bit."""
     from videosys_b200.models.transformers.open_sora_plan_v110_transformer_3d import rope_tables
 
-    M = ref_loader.load_osp_v110()
     D, Hh, h, w, Fr = 72, 3, 5, 7, 9
+    want2, want1 = pin[f"osp_rope.{PC.DT[dtype]}"]
     q2 = synth.normalish("rope.q2", (2, Hh, h * w, D)).to(dtype)
-    pos2 = M.PositionGetter2D()(2, h, w, "cpu")
-    want2 = M.LinearScalingRoPE2D(scaling_factor=2)(q2, pos2)
     yx = torch.cartesian_prod(torch.arange(h), torch.arange(w))
     c, s, half = rope_tables(D, [yx[:, 0], yx[:, 1]], 2, dtype, "cpu")
     assert half == 18
@@ -381,58 +240,41 @@ def test_osp_v110_rope_tables_vs_reference_classes(dtype):
         partner = q.reshape(*q.shape[:-1], D // (2 * half), 2, half).flip(-2).reshape(q.shape)
         return q * c.to(dtype) + partner * s.to(dtype)
 
-    assert torch.equal(apply(q2, c, s, half), want2)
+    pins.assert_exact(apply(q2, c, s, half), want2, "2-D")
     q1 = synth.normalish("rope.q1", (4, Hh, Fr, D)).to(dtype)
-    want1 = M.LinearScalingRoPE1D(scaling_factor=2)(q1, M.PositionGetter1D()(4, Fr, "cpu"))
     c, s, half = rope_tables(D, [torch.arange(Fr)], 2, dtype, "cpu")
-    assert half == 36 and torch.equal(apply(q1, c, s, half), want1)
+    assert half == 36
+    pins.assert_exact(apply(q1, c, s, half), want1, "1-D")
 
 
 # ---- Latte: oracle and product host logic against the UNMODIFIED reference model ---------------------------------------------
-LATTE_SMALL = dict(num_attention_heads=2, attention_head_dim=72, in_channels=4, out_channels=8, num_layers=2,
-                   cross_attention_dim=144, attention_bias=True, sample_size=8, patch_size=2, activation_fn="gelu-approximate",
-                   norm_type="ada_norm_single", norm_elementwise_affine=False, norm_eps=1e-6, caption_channels=32, video_length=6)
-LATTE_SMALL_O = dict(heads=2, head_dim=72, layers=2, patch=2, sample_size=8, out_channels=8, video_length=6)
 
 
-def _latte_ref(dtype=torch.float32, tag="lattep."):
-    ref = ref_loader.build_latte(dtype=dtype, **LATTE_SMALL)
-    sd = synth.fill_state_dict({k: v.float() for k, v in ref.state_dict().items()}, tag)
-    sd = {k: v.to(dtype) for k, v in sd.items()}
-    ref.load_state_dict(sd)
-    return ref, sd
+def _latte_sd(pin, dtype=torch.float32):
+    return {k: v.to(dtype) for k, v in _fill(pin, f"latte.{PC.DT[dtype]}", "lattep.").items()}
 
 
-def _latte_call(ref, x, t, enc, all_ts=(900, 500)):
-    return ref(x, timestep=t, all_timesteps=torch.tensor(list(all_ts)), encoder_hidden_states=enc,
-               added_cond_kwargs={"resolution": None, "aspect_ratio": None}, enable_temporal_attentions=True,
-               return_dict=False)[0]
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_latte_oracle_vs_reference_model(dtype):
+def test_latte_oracle_vs_reference_model(pin, dtype):
     """oracle/latte_oracle.transformer_forward against the reference's own LatteT2V (models/transformers/
-    latte_transformer_3d.py, executed unmodified; its diffusers leaves = the reference's vendored copies, ref_loader.load_latte):
-    the whole forward -- PatchEmbed + 2-D sin-cos table, AdaLayerNormSingle, caption projection, both block kinds,
-    temp_pos_embed, output head, un-patchify.  fp32: equal up to summation order; bf16: bit for bit."""
+    latte_transformer_3d.py): the whole forward -- PatchEmbed + 2-D sin-cos table, AdaLayerNormSingle, caption projection,
+    both block kinds, temp_pos_embed, output head, un-patchify.  fp32: equal up to summation order; bf16: bit for bit."""
     from oracle import latte_oracle as LO
 
-    ref, sd = _latte_ref(dtype)
+    sd = _latte_sd(pin, dtype)
     x = synth.normalish("lattep.x", (2, 4, 6, 8, 8)).to(dtype)
     enc = synth.normalish("lattep.enc", (2, 7, 32)).to(dtype)
-    t = torch.tensor([500, 500])
     with torch.no_grad():
-        want = _latte_call(ref, x, t, enc)
-        got = LO.transformer_forward(sd, LATTE_SMALL_O, x, t, enc)
-    assert got.shape == want.shape
+        got = LO.transformer_forward(sd, PC.LATTE_SMALL_O, x, torch.tensor([500, 500]), enc)
     if dtype == torch.float32:
-        assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
+        pins.assert_close(got, pin["latte.float32"], rtol=1e-4, atol=1e-5)
     else:
-        print(f"[pin] latte oracle bf16 vs reference bf16: bit-equal {(got == want).float().mean().item()*100:.1f} %")
-        assert torch.equal(got, want)
+        pins.assert_exact(got, pin["latte.bfloat16"], "latte oracle bf16")
 
 
-def test_latte_mirror_vs_reference_model(monkeypatch):
+def test_latte_mirror_vs_reference_model(pin, monkeypatch):
     """videosys_b200's LatteT2V (kernel entries = torch stand-ins) against the reference model, fp32, incl. 8 PAB steps with the
     MLP skip on both sides."""
     from tests import kernels_emul
@@ -440,83 +282,55 @@ def test_latte_mirror_vs_reference_model(monkeypatch):
     from videosys_b200.models.transformers.latte_transformer_3d import LatteT2V
 
     kernels_emul.emulate(monkeypatch)
-    ref, sd = _latte_ref()
-    net = LatteT2V(**LATTE_SMALL)
-    net.load_state_dict(sd)
+    net = LatteT2V(**PC.LATTE_SMALL)
+    net.load_state_dict(_latte_sd(pin))
     net.eval()
     x = synth.normalish("lattep.x", (2, 4, 6, 8, 8))
     enc = synth.normalish("lattep.enc", (2, 7, 32))
-    t = torch.tensor([500, 500])
-    with torch.no_grad():
-        want = _latte_call(ref, x, t, enc)
-    got = net(x, timestep=t, all_timesteps=[900, 500], encoder_hidden_states=enc, return_dict=False)[0]
-    assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
-    P = ref_loader.load().pab_mgr
-    ts = [900, 700, 650, 600, 550, 500, 450, 50]
-    mlp = {700: {"block": [0, 1], "skip_count": 2}, 550: {"block": [1], "skip_count": 1}}
-    kw = dict(spatial_broadcast=True, spatial_threshold=[100, 800], spatial_range=2, temporal_broadcast=True,
-              temporal_threshold=[100, 800], temporal_range=3, cross_broadcast=True, cross_threshold=[100, 800], cross_range=6,
-              mlp_broadcast=True, mlp_spatial_broadcast_config=mlp, mlp_temporal_broadcast_config=mlp)
-    P.set_pab_manager(P.PABConfig(**kw))
-    P.update_steps(len(ts))
-    ours.set_pab_manager(ours.PABConfig(**kw))
-    ours.update_steps(len(ts))
+    got = net(x, timestep=torch.tensor([500, 500]), all_timesteps=[900, 500], encoder_hidden_states=enc, return_dict=False)[0]
+    pins.assert_close(got, pin["latte.float32"], rtol=1e-4, atol=1e-5)
+    ours.set_pab_manager(ours.PABConfig(**PC.LATTE_PAB_KW))
+    ours.update_steps(len(PC.PAB_TS))
     net.reset_pab_state()
     try:
-        for step, tv in enumerate(ts):
+        for step, tv in enumerate(PC.PAB_TS):
             x = synth.normalish(f"lattep.x{step}", (2, 4, 6, 8, 8))
-            tt = torch.tensor([tv, tv])
-            with torch.no_grad():
-                want = _latte_call(ref, x, tt, enc, ts)
-            got = net(x, timestep=tt, all_timesteps=ts, encoder_hidden_states=enc, return_dict=False)[0]
-            assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (step, (got - want).abs().max())
+            got = net(x, timestep=torch.tensor([tv, tv]), all_timesteps=PC.PAB_TS, encoder_hidden_states=enc, return_dict=False)[0]
+            pins.assert_close(got, pin[f"latte.pab.{step}"], rtol=1e-4, atol=1e-5, what=step)
     finally:
-        P.PAB_MANAGER = None
         ours.set_pab_manager(None)
 
 
 # ---- CogVideoX: oracle and product host logic against the UNMODIFIED reference model ------------------------------------------
-COGX_SMALL = dict(num_attention_heads=4, attention_head_dim=64, in_channels=4, out_channels=4, time_embed_dim=64, text_embed_dim=48,
-                  num_layers=2, sample_width=16, sample_height=12, sample_frames=9, max_text_seq_length=16)
-COGX_SMALL_O = dict(heads=4, head_dim=64, layers=2, patch=2, max_text=16, sample_width=16, sample_height=12, sample_frames=9,
-                    out_channels=4)
 
 
-def _cogx_ref(dtype=torch.float32, tag="cogxp."):
-    ref = ref_loader.build_cogvideox(dtype=dtype, **COGX_SMALL)
-    sd = synth.fill_state_dict({k: v.float() for k, v in ref.state_dict().items()}, tag)
-    for k in sd:  # LayerNorm weights around 1 (fill_state_dict treats them as matrices)
-        if k.endswith("norm.weight") or k.endswith("norm_final.weight") or k.endswith("norm_q.weight") or k.endswith("norm_k.weight"):
-            sd[k] = 1.0 + 0.2 * synth.uniform(tag + k, tuple(sd[k].shape))
-    sd = {k: v.to(dtype) for k, v in sd.items()}
-    ref.load_state_dict(sd)
-    return ref, sd
+def cogx_weights(pin, key, tag, dtype):
+    """synth weights for the reference's CogVideoX state dict (fp32 template), LayerNorm weights around 1 (fill_state_dict
+    treats them as matrices), cast to dtype."""
+    return PC.cogx_norms(_fill(pin, key, tag), tag, dtype)
+
+
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16, torch.float16])
-def test_cogvideox_oracle_vs_reference_model(dtype):
-    """oracle/cogvideox_oracle.transformer_forward against the reference's own CogVideoXTransformer3DModel (executed
-    unmodified; diffusers Attention / FeedForward = the reference's vendored copies, ref_loader.load_cogvideox): patch / text
+def test_cogvideox_oracle_vs_reference_model(pin, dtype):
+    """oracle/cogvideox_oracle.transformer_forward against the reference's own CogVideoXTransformer3DModel: patch / text
     embedding, position table, LayerNormZero blocks with the joint-attention processor, norm_final + AdaLayerNorm head,
     un-patchify."""
     from oracle import cogvideox_oracle as CO
 
-    ref, sd = _cogx_ref(dtype)
+    sd = cogx_weights(pin, f"cogxp.{PC.DT[dtype]}", "cogxp.", dtype)
     lat = synth.normalish("cogxp.lat", (2, 3, 4, 12, 16)).to(dtype)
     txt = synth.normalish("cogxp.txt", (2, 16, 48)).to(dtype)
-    ts = torch.tensor([499, 499])
     with torch.no_grad():
-        want = ref(lat, txt, ts, return_dict=False)[0]
-        got = CO.transformer_forward(sd, COGX_SMALL_O, lat, txt, ts)
-    assert got.shape == want.shape
+        got = CO.transformer_forward(sd, PC.COGX_SMALL_O, lat, txt, torch.tensor([499, 499]))
     if dtype == torch.float32:
-        assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
+        pins.assert_close(got, pin["cogx.float32"], rtol=1e-4, atol=1e-5)
     else:
-        print(f"[pin] cogvideox oracle {dtype} vs reference: bit-equal {(got == want).float().mean().item()*100:.1f} %")
-        assert torch.equal(got, want)
+        pins.assert_exact(got, pin[f"cogx.{PC.DT[dtype]}"], f"cogvideox oracle {dtype}")
 
 
-def test_cogvideox_mirror_vs_reference_model(monkeypatch):
+def test_cogvideox_mirror_vs_reference_model(pin, monkeypatch):
     """videosys_b200's CogVideoXTransformer3DModel (kernel entries = torch stand-ins) against the reference model, fp32, plain
     and over 8 PAB steps."""
     from tests import kernels_emul
@@ -524,81 +338,64 @@ def test_cogvideox_mirror_vs_reference_model(monkeypatch):
     from videosys_b200.models.transformers.cogvideox_transformer_3d import CogVideoXTransformer3DModel
 
     kernels_emul.emulate(monkeypatch)
-    ref, sd = _cogx_ref()
-    net = CogVideoXTransformer3DModel(**COGX_SMALL)
+    sd = cogx_weights(pin, "cogxp.float32", "cogxp.", torch.float32)
+    net = CogVideoXTransformer3DModel(**PC.COGX_SMALL)
     missing, unexpected = net.load_state_dict(sd, strict=False)
     assert not missing and all(".attn1.to_" in k and ("_temp" in k or "_cross" in k or "_context" in k or "temporal" in k)
                                for k in unexpected), (missing, unexpected)  # the vendored Attention's Vchitect-only members
     net.eval()
     lat = synth.normalish("cogxp.lat", (2, 3, 4, 12, 16))
     txt = synth.normalish("cogxp.txt", (2, 16, 48))
-    ts = torch.tensor([499, 499])
-    with torch.no_grad():
-        want = ref(lat, txt, ts, return_dict=False)[0]
-    got = net(lat, txt, ts, return_dict=False)[0]
-    assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
-    P = ref_loader.load().pab_mgr
-    kw = dict(spatial_broadcast=True, spatial_threshold=[100, 850], spatial_range=2)
-    steps = [900, 700, 650, 600, 550, 500, 450, 50]
-    P.set_pab_manager(P.PABConfig(**kw))
-    P.update_steps(len(steps))
-    ours.set_pab_manager(ours.PABConfig(**kw))
-    ours.update_steps(len(steps))
+    got = net(lat, txt, torch.tensor([499, 499]), return_dict=False)[0]
+    pins.assert_close(got, pin["cogx.float32"], rtol=1e-4, atol=1e-5)
+    ours.set_pab_manager(ours.PABConfig(**PC.COGX_PAB_KW))
+    ours.update_steps(len(PC.PAB_TS))
     net.reset_pab_state()
     try:
-        for step, tv in enumerate(steps):
+        for step, tv in enumerate(PC.PAB_TS):
             lat = synth.normalish(f"cogxp.lat{step}", (2, 3, 4, 12, 16))
-            tt = torch.tensor([tv, tv])
-            with torch.no_grad():
-                want = ref(lat, txt, tt, return_dict=False)[0]
-            got = net(lat, txt, tt, return_dict=False)[0]
-            assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (step, (got - want).abs().max())
+            got = net(lat, txt, torch.tensor([tv, tv]), return_dict=False)[0]
+            pins.assert_close(got, pin[f"cogx.pab.{step}"], rtol=1e-4, atol=1e-5, what=step)
     finally:
-        P.PAB_MANAGER = None
         ours.set_pab_manager(None)
 
 
 # ---- Vchitect: oracle and product host logic against the UNMODIFIED reference transformer ---------------------------------------
-VCH_SMALL = dict(sample_size=8, patch_size=2, in_channels=4, num_layers=3, attention_head_dim=64, num_attention_heads=2,
-                 joint_attention_dim=48, caption_projection_dim=128, pooled_projection_dim=40, out_channels=4, pos_embed_max_size=12)
-VCH_SMALL_O = dict(heads=2, head_dim=64, layers=3, patch=2, sample_size=8, pos_embed_max_size=12, out_channels=4)
 
 
-def _vch_ref(dtype=torch.float32, tag="vchm."):
-    ref = ref_loader.build_vchitect(dtype=dtype, **VCH_SMALL)
-    sd0 = {k: v.float() for k, v in ref.state_dict().items()}
-    sd = synth.fill_state_dict(sd0, tag)
-    sd["pos_embed.pos_embed"] = sd0["pos_embed.pos_embed"]  # the sin-cos table is not a weight
-    sd = {k: v.to(dtype) for k, v in sd.items()}
-    ref.load_state_dict(sd)
-    return ref, sd
+def _vch_sd(pin, dtype=torch.float32):
+    """The reference's weights: synth fill of its state dict, its own sin-cos position table kept (not a weight; the product
+    module builds the same table, checked bit for bit against the reference's)."""
+    from videosys_b200.models.transformers.vchitect_transformer_3d import VchitectXLTransformerModel
+
+    table = VchitectXLTransformerModel(**PC.VCH_SMALL).state_dict()["pos_embed.pos_embed"].float()
+    pins.assert_exact(table.to(dtype), pin[f"vchm.pos_embed.{PC.DT[dtype]}"], "position table")
+    sd = _fill(pin, f"vchm.{PC.DT[dtype]}", "vchm.")
+    sd["pos_embed.pos_embed"] = table
+    return {k: v.to(dtype) for k, v in sd.items()}
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize("Fr", [5, 1])
-def test_vchitect_oracle_vs_reference_model(Fr, dtype):
+def test_vchitect_oracle_vs_reference_model(pin, Fr, dtype):
     """oracle/vchitect_oracle.transformer_forward against the reference's VchitectXLTransformerModel (vchitect_transformer_3d.py
-    executed unmodified on the reference's VchitectAttention; five diffusers leaf classes restated in oracle/ref_loader.py):
-    per-frame text broadcast in the first block, context_pre_only last block, the three attentions, norm_out, un-patchify."""
+    on the reference's VchitectAttention): per-frame text broadcast in the first block, context_pre_only last block, the three
+    attentions, norm_out, un-patchify."""
     from oracle import vchitect_oracle as VO
 
-    ref, sd = _vch_ref(dtype)
+    sd = _vch_sd(pin, dtype)
     lat = synth.normalish("vchm.lat", (1, Fr, 4, 12, 16)).to(dtype)
     enc = synth.normalish("vchm.enc", (1, 9, 48)).to(dtype)
     pooled = synth.normalish("vchm.pool", (1, 40)).to(dtype)
-    ts = torch.tensor([500.0])
     with torch.no_grad():
-        want = ref(lat, encoder_hidden_states=enc, pooled_projections=pooled, timestep=ts, return_dict=False)[0]
-        got = VO.transformer_forward(sd, VCH_SMALL_O, lat, enc, pooled, ts)
-    assert got.shape == want.shape
+        got = VO.transformer_forward(sd, PC.VCH_SMALL_O, lat, enc, pooled, torch.tensor([500.0]))
     if dtype == torch.float32:
-        assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
+        pins.assert_close(got, pin[f"vch.{Fr}.float32"], rtol=1e-4, atol=1e-5)
     else:
-        print(f"[pin] vchitect oracle bf16 vs reference: bit-equal {(got == want).float().mean().item()*100:.1f} %")
-        assert torch.equal(got, want)
+        pins.assert_exact(got, pin[f"vch.{Fr}.bfloat16"], "vchitect oracle bf16")
 
 
-def test_vchitect_mirror_vs_reference_model(monkeypatch):
+def test_vchitect_mirror_vs_reference_model(pin, monkeypatch):
     """videosys_b200's VchitectXLTransformerModel (kernel entries = torch stand-ins) against the reference model: strict
     state-dict compatibility, fp32 forward, and 8 steps with the three PAB gates on both sides."""
     from tests import kernels_emul
@@ -606,40 +403,30 @@ def test_vchitect_mirror_vs_reference_model(monkeypatch):
     from videosys_b200.models.transformers.vchitect_transformer_3d import VchitectXLTransformerModel
 
     kernels_emul.emulate(monkeypatch)
-    ref, sd = _vch_ref()
-    net = VchitectXLTransformerModel(**VCH_SMALL)
-    net.load_state_dict(sd)  # strict
+    net = VchitectXLTransformerModel(**PC.VCH_SMALL)
+    net.load_state_dict(_vch_sd(pin))  # strict
     net.eval()
     enc = synth.normalish("vchm.enc", (1, 9, 48))
     pooled = synth.normalish("vchm.pool", (1, 40))
-    P = ref_loader.load().pab_mgr
-    kw = dict(spatial_broadcast=True, spatial_threshold=[100, 800], spatial_range=2, temporal_broadcast=True,
-              temporal_threshold=[100, 800], temporal_range=3, cross_broadcast=True, cross_threshold=[100, 800], cross_range=4)
     for pab in (False, True):
-        steps = [900, 700, 650, 600, 550, 500, 450, 50] if pab else [500]
+        steps = PC.PAB_TS if pab else [500]
         if pab:
-            P.set_pab_manager(P.PABConfig(**kw))
-            P.update_steps(len(steps))
-            ours.set_pab_manager(ours.PABConfig(**kw))
+            ours.set_pab_manager(ours.PABConfig(**PC.VCH_PAB_KW))
             ours.update_steps(len(steps))
             net.reset_pab_state()
         try:
             for step, tv in enumerate(steps):
                 lat = synth.normalish(f"vchm.lat{step}", (1, 4, 4, 12, 16))
-                ts = torch.tensor([float(tv)])
-                with torch.no_grad():
-                    want = ref(lat, encoder_hidden_states=enc, pooled_projections=pooled, timestep=ts, return_dict=False)[0]
-                got = net(lat, enc, pooled, ts, return_dict=False)[0]
-                assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (pab, step, (got - want).abs().max())
+                got = net(lat, enc, pooled, torch.tensor([float(tv)]), return_dict=False)[0]
+                pins.assert_close(got, pin[f"vch.mirror.{int(pab)}.{step}"], rtol=1e-4, atol=1e-5, what=(pab, step))
         finally:
-            P.PAB_MANAGER = None
             ours.set_pab_manager(None)
 
 
-def _vch_sp_worker(rank, world, port, Fr, q):
-    import os
+
+
+def _vch_sp_worker(rank, world, port, Fr, sd, q):
     import traceback
-    import types
 
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
@@ -661,214 +448,134 @@ def _vch_sp_worker(rank, world, port, Fr, q):
                 o.copy_(r)
 
         dist.all_to_all = a2a
-        RC = ref_loader.load().comm
-
-        def gather_cpu(input_, pg, dim, pad):  # the reference's _gather_sequence_func (comm.py:170-190) minus its CUDA assert
-            parts = [torch.empty_like(input_.contiguous()) for _ in range(dist.get_world_size(pg))]
-            dist.all_gather(parts, input_.contiguous(), group=pg)
-            out = torch.cat(parts, dim=dim)
-            return out.narrow(dim, 0, out.size(dim) - pad) if pad > 0 else out
-
-        RC._gather_sequence_func = gather_cpu
-        ref, sd = _vch_ref()
-        pm = types.SimpleNamespace(sp_size=world, sp_group=dist.group.WORLD, cp_size=1, sp_rank=rank)
-        ref.parallel_manager = pm
-        for mod in ref.modules():
-            if hasattr(mod, "parallel_manager"):
-                mod.parallel_manager = pm
-        net = VchitectXLTransformerModel(**VCH_SMALL)
-        net.load_state_dict(sd)
+        net = VchitectXLTransformerModel(**PC.VCH_SMALL)
+        net.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
         net.eval()
         net.enable_parallel(1, world, False)
-        lat = synth.normalish("vchsp.lat", (1, Fr, 4, 12, 16))
-        enc = synth.normalish("vchsp.enc", (1, 9, 48))
-        pooled = synth.normalish("vchsp.pool", (1, 40))
-        ts = torch.tensor([500.0])
-        with torch.no_grad():
-            want = ref(lat, encoder_hidden_states=enc, pooled_projections=pooled, timestep=ts, return_dict=False)[0]
-        got = net(lat, enc, pooled, ts, return_dict=False)[0]
-        q.put((rank, float((got - want).abs().max()), float(want.abs().max()), tuple(got.shape) == tuple(want.shape), None))
+        lat, enc, pooled = PC.vch_sp_inputs(Fr)
+        got = net(lat, enc, pooled, torch.tensor([500.0]), return_dict=False)[0]
+        q.put((rank, got.detach().numpy(), None))
         dist.barrier()
         dist.destroy_process_group()
     except Exception:  # pragma: no cover
-        q.put((rank, None, None, None, traceback.format_exc()))
+        q.put((rank, None, traceback.format_exc()))
 
 
 @pytest.mark.parametrize("Fr", [4, 5, 2])  # 5 frames: a zero frame pads the last rank; 2: one frame per rank (temporal branch * 0)
-def test_vchitect_sequence_parallel_vs_reference_gloo_world2(Fr):
-    """Two gloo ranks, both running the UNMODIFIED reference transformer and videosys_b200's (kernel entries = torch stand-ins)
-    under frame-sharded sequence parallelism: same output on every rank, incl. the reference's quirks under sp (cross attention
-    against the text keys of the rank's own first frame, cur_frame == 1 judged on the local frame count)."""
+def test_vchitect_sequence_parallel_vs_reference_gloo_world2(pin, monkeypatch, Fr):
+    """Two gloo ranks running videosys_b200's transformer (kernel entries = torch stand-ins) under frame-sharded sequence
+    parallelism against what the UNMODIFIED reference transformer computed on every rank under the same sharding, incl. the
+    reference's quirks under sp (cross attention against the text keys of the rank's own first frame, cur_frame == 1 judged
+    on the local frame count)."""
     import multiprocessing as mp
-    import os
 
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")  # CPU ranks on gloo: with a GPU visible, initialize() picks NCCL
     world, port = 2, 30700 + (os.getpid() % 250) + Fr
+    sd = {k: v.numpy() for k, v in _vch_sd(pin).items()}  # by value: no shared-memory handles that die with the worker
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
-    procs = [ctx.Process(target=_vch_sp_worker, args=(r, world, port, Fr, q)) for r in range(world)]
+    procs = [ctx.Process(target=_vch_sp_worker, args=(r, world, port, Fr, sd, q)) for r in range(world)]
     [p.start() for p in procs]
+    recs = pin[f"vch.sp.{Fr}"]
     for _ in range(world):
-        r, err_abs, scale, same_shape, tb = q.get(timeout=300)
+        r, got, tb = q.get(timeout=300)
         assert tb is None, tb
-        assert same_shape and err_abs <= 1e-4 * max(scale, 1.0), (r, err_abs, scale)
+        pins.assert_close(torch.from_numpy(got), recs[r], rtol=0.0, atol=1e-4 * max(recs[r]["max_abs"], 1.0), what=r)
     [p.join(timeout=60) for p in procs]
 
 
 # ---- Open-Sora-Plan v1.2.0: the product's host logic against the UNMODIFIED reference model --------------------------------
-OSP12_SMALL = dict(num_attention_heads=2, attention_head_dim=96, in_channels=4, out_channels=8, num_layers=2, cross_attention_dim=192,
-                   attention_bias=True, sample_size=(8, 8), sample_size_t=5, patch_size=2, patch_size_t=1,
-                   activation_fn="gelu-approximate", norm_type="ada_norm_single", norm_elementwise_affine=False, norm_eps=1e-6,
-                   caption_channels=32, interpolation_scale_h=1.0, interpolation_scale_w=2.0, interpolation_scale_t=1.5,
-                   attention_mode="math", downsampler=None, use_rope=True)
 
 
-def _osp12_pair(cfg, tag="osp12."):
+
+
+def _osp12_net(pin, cfg, key, tag):
     from videosys_b200.models.transformers.open_sora_plan_v120_transformer_3d import OpenSoraT2V
 
-    ref = ref_loader.build_osp_v120(**cfg)
-    sd = synth.fill_state_dict(ref.state_dict(), tag)
-    ref.load_state_dict(sd)
     net = OpenSoraT2V(**cfg)
-    net.load_state_dict(sd)  # strict
-    return ref, net.eval()
+    net.load_state_dict(_fill(pin, key, tag))  # strict
+    return net.eval()
 
 
-def _osp12_call(ref, x, t, enc, m):
-    return ref(x, timestep=t, encoder_hidden_states=enc, attention_mask=torch.ones(x.shape[0], x.shape[2], x.shape[3], x.shape[4]),
-               encoder_attention_mask=m, return_dict=False)[0]
-
-
-@pytest.mark.parametrize("use_rope,HW", [(True, (8, 8)), (False, (8, 8)), (True, (12, 8))])
-def test_osp_v120_mirror_vs_reference_model(monkeypatch, use_rope, HW):
-    """videosys_b200's OpenSoraT2V (kernel entries = torch stand-ins) against the reference's own OpenSoraT2V executed
-    unmodified: RoPE3D tables with per-axis interpolation scales, absolute position tables when RoPE is off, text padding
-    mask, block order, output head / un-patchify."""
+@pytest.mark.parametrize("use_rope,HW", PC.OSP12_MIRROR_CASES)
+def test_osp_v120_mirror_vs_reference_model(pin, monkeypatch, use_rope, HW):
+    """videosys_b200's OpenSoraT2V (kernel entries = torch stand-ins) against the reference's own OpenSoraT2V: RoPE3D tables
+    with per-axis interpolation scales, absolute position tables when RoPE is off, text padding mask, block order, output
+    head / un-patchify."""
     from tests import kernels_emul
 
     kernels_emul.emulate(monkeypatch)
-    ref, net = _osp12_pair(dict(OSP12_SMALL, use_rope=use_rope))
-    x, enc, m = _osp_inputs(2, 5, HW, tag="osp12.")
-    t = torch.tensor([500, 500])
-    with torch.no_grad():
-        want = _osp12_call(ref, x, t, enc, m)
-    got = net(x, timestep=t, encoder_hidden_states=enc, encoder_attention_mask=m, return_dict=False)[0]
-    assert got.shape == want.shape
-    assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
+    key = PC.osp12_key(use_rope, HW)
+    net = _osp12_net(pin, dict(PC.OSP12_SMALL, use_rope=use_rope), key, "osp12.")
+    x, enc, m = PC.osp_inputs(2, 5, HW, tag="osp12.")
+    got = net(x, timestep=torch.tensor([500, 500]), encoder_hidden_states=enc, encoder_attention_mask=m, return_dict=False)[0]
+    pins.assert_close(got, pin[key], rtol=1e-4, atol=1e-5)
 
 
-def test_osp_v120_pab_vs_reference_model(monkeypatch):
+def test_osp_v120_pab_vs_reference_model(pin, monkeypatch):
     from tests import kernels_emul
     from videosys_b200.core.pab import pab_mgr as ours
 
     kernels_emul.emulate(monkeypatch)
-    P = ref_loader.load().pab_mgr
-    ref, net = _osp12_pair(OSP12_SMALL, "osp12p.")
-    ts = [900, 700, 650, 600, 550, 500, 450, 50]
-    kw = dict(spatial_broadcast=True, spatial_threshold=[100, 850], spatial_range=2, cross_broadcast=True,
-              cross_threshold=[100, 850], cross_range=3)
-    P.set_pab_manager(P.PABConfig(**kw))
-    P.update_steps(len(ts))
-    ours.set_pab_manager(ours.PABConfig(**kw))
-    ours.update_steps(len(ts))
+    net = _osp12_net(pin, PC.OSP12_SMALL, "osp12p", "osp12p.")
+    ours.set_pab_manager(ours.PABConfig(**PC.OSP12_PAB_KW))
+    ours.update_steps(len(PC.PAB_TS))
     net.reset_pab_state()
     try:
-        for step, t in enumerate(ts):
-            x, enc, m = _osp_inputs(2, 5, (8, 8), tag=f"osp12p{step}.")
-            tt = torch.tensor([t, t])
-            with torch.no_grad():
-                want = _osp12_call(ref, x, tt, enc, m)
-            got = net(x, timestep=tt, encoder_hidden_states=enc, encoder_attention_mask=m, return_dict=False)[0]
-            assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (step, (got - want).abs().max())
+        for step, t in enumerate(PC.PAB_TS):
+            x, enc, m = PC.osp_inputs(2, 5, (8, 8), tag=f"osp12p{step}.")
+            got = net(x, timestep=torch.tensor([t, t]), encoder_hidden_states=enc, encoder_attention_mask=m, return_dict=False)[0]
+            pins.assert_close(got, pin[f"osp12p.{step}"], rtol=1e-4, atol=1e-5, what=step)
     finally:
-        P.PAB_MANAGER = None
         ours.set_pab_manager(None)
 
 
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16, torch.float32])
-def test_osp_v120_rope3d_tables_vs_reference_class(dtype):
+def test_osp_v120_rope3d_tables_vs_reference_class(pin, dtype):
     from videosys_b200.models.transformers.open_sora_plan_v120_transformer_3d import rope3d_tables
 
-    M = ref_loader.load_osp_v120()
     D, Hh, T, h, w = 96, 3, 4, 3, 5
     q = synth.normalish("rope3.q", (2, Hh, T * h * w, D)).to(dtype)
-    pos = M.PositionGetter3D()(2, T, h, w, "cpu")
-    want = M.RoPE3D(interpolation_scale_thw=(1.5, 1.0, 2.0))(q, pos)
     c, s, half = rope3d_tables(D, T, h, w, (1.5, 1.0, 2.0), dtype, "cpu")
     assert half == 16
     partner = q.reshape(*q.shape[:-1], D // (2 * half), 2, half).flip(-2).reshape(q.shape)
-    assert torch.equal(q * c.to(dtype) + partner * s.to(dtype), want)
+    pins.assert_exact(q * c.to(dtype) + partner * s.to(dtype), pin[f"osp12_rope3d.{PC.DT[dtype]}"])
 
 
-def test_stdit3_mirror_vs_reference_model(monkeypatch):
+
+
+
+
+def test_stdit3_mirror_vs_reference_model(pin, monkeypatch):
     """The headline model's front end (videosys_b200 STDiT3, kernel entries = torch stand-ins, bf16 as it insists) against
-    the reference STDiT3 executed unmodified: within the reference's own bf16-vs-fp32 error, with PAB off and over 6 PAB
-    steps (hoisted text projections, modulation tables, per-frame mask select, final layer on the shard, un-patchify)."""
+    the reference STDiT3: within the reference's own bf16-vs-fp32 error, with PAB off and over 6 PAB steps (hoisted text
+    projections, modulation tables, per-frame mask select, final layer on the shard, un-patchify)."""
     from tests import kernels_emul
     from videosys_b200.core.pab import pab_mgr as ours
     from videosys_b200.models.transformers.open_sora_transformer_3d import STDiT3, STDiT3Config
 
     kernels_emul.emulate(monkeypatch)
     c = cases.small_model_cfg(depth=2)
-    ref16 = ref_loader.build_stdit3(dtype=torch.bfloat16, **c)
-    sd = synth.fill_state_dict(ref16.state_dict(), "stde.")
-    ref16.load_state_dict(sd)
-    ref32 = ref_loader.build_stdit3(dtype=torch.float32, **c)
-    ref32.load_state_dict({k: v.float() for k, v in sd.items()})
     net = STDiT3(STDiT3Config(**c)).to(torch.bfloat16)
-    net.load_state_dict(sd)
+    net.load_state_dict(_fill(pin, "stde.bfloat16", "stde."))
     net.eval()
-    P = ref_loader.load().pab_mgr
-
-    def rel(a, b):
-        return ((a.double() - b.double()).norm() / b.double().norm()).item()
-
-    def run(model, inp, dt):
-        f = lambda v: v.to(dt) if torch.is_tensor(v) and v.is_floating_point() else v  # noqa: E731
-        with torch.no_grad():
-            return model(f(inp["x"]), f(inp["timestep"]), f(inp["y"]), mask=inp["mask"], x_mask=inp["x_mask"], fps=f(inp["fps"]),
-                         height=f(inp["height"]), width=f(inp["width"]))
-
     inp = cases.forward_inputs(torch.bfloat16)
-    got, w16, w32 = run(net, inp, torch.bfloat16), run(ref16, inp, torch.bfloat16), run(ref32, inp, torch.float32)
-    assert got.shape == w32.shape and rel(got, w32) <= 1.3 * rel(w16, w32) + 1e-4, (rel(got, w32), rel(w16, w32))
-    kw = dict(spatial_broadcast=True, spatial_threshold=[100, 930], spatial_range=2, temporal_broadcast=True,
-              temporal_threshold=[100, 930], temporal_range=3, cross_broadcast=True, cross_threshold=[100, 930], cross_range=4)
-    steps = [900.0, 800.0, 700.0, 600.0, 500.0, 50.0]
-    ours.set_pab_manager(ours.PABConfig(**kw))
-    ours.update_steps(len(steps))
+    pins.assert_rel(PC.stdit3_run(net, inp, torch.bfloat16), pin["stde.0"], "PAB off")
+    ours.set_pab_manager(ours.PABConfig(**PC.STDIT3_PAB_KW))
+    ours.update_steps(len(PC.STDIT3_PAB_TS))
     net.reset_pab_state()
     try:
-        outs = []
-        for t in steps:
+        for i, t in enumerate(PC.STDIT3_PAB_TS):
             inp["timestep"] = torch.tensor([t, t], dtype=torch.bfloat16)
-            outs.append(run(net, inp, torch.bfloat16))
-        for model, dt, name in ((ref16, torch.bfloat16, "w16"), (ref32, torch.float32, "w32")):
-            P.set_pab_manager(P.PABConfig(**kw))
-            P.update_steps(len(steps))
-            res = []
-            for t in steps:
-                inp["timestep"] = torch.tensor([t, t], dtype=torch.bfloat16)
-                res.append(run(model, inp, dt))
-            P.PAB_MANAGER = None
-            if name == "w16":
-                r16 = res
-            else:
-                r32 = res
-        for i in range(len(steps)):
-            assert rel(outs[i], r32[i]) <= 1.3 * rel(r16[i], r32[i]) + 1e-4, (i, rel(outs[i], r32[i]), rel(r16[i], r32[i]))
+            pins.assert_rel(PC.stdit3_run(net, inp, torch.bfloat16), pin[f"stde.{i + 1}"], i)
     finally:
-        P.PAB_MANAGER = None
         ours.set_pab_manager(None)
 
 
 # ---- CogVideoX-5b: rotary position embeddings ------------------------------------------------------------------------------------
-def _cogx_rotary(T=3, gh=6, gw=8, D=64):
-    from oracle import cogvideox_oracle as CO
-
-    return CO.rotary_3d(D, CO.resize_crop_region_for_grid((gh, gw), 45, 30), (gh, gw), T)
 
 
-def test_cogvideox_rotary_helpers_vs_reference():
+def test_cogvideox_rotary_helpers_vs_reference(pin):
     """oracle rotary_3d / resize_crop_region_for_grid / apply_rotary_emb and the pipeline mirror's
     _prepare_rotary_positional_embeddings against the reference's own functions (models/modules/embeddings.py:283-412,
     pipelines/cogvideox/pipeline_cogvideox.py:758-773 -- the pipeline module itself needs diffusers: its crop helper is
@@ -876,55 +583,45 @@ def test_cogvideox_rotary_helpers_vs_reference():
     from oracle import cogvideox_oracle as CO
     from videosys_b200.pipelines.cogvideox.pipeline_cogvideox import CogVideoXPipeline
 
-    ref_loader.load_cogvideox()
-    import importlib
-
-    E = importlib.import_module("videosys.models.modules.embeddings")
-    for (gh, gw) in ((30, 45), (6, 8), (20, 20), (9, 40)):
-        crops = CO.resize_crop_region_for_grid((gh, gw), 45, 30)
-        rc, rs = E.get_3d_rotary_pos_embed(64, crops, (gh, gw), 5, use_real=True)
-        oc, os_ = CO.rotary_3d(64, crops, (gh, gw), 5)
-        assert torch.equal(rc, oc) and torch.equal(rs, os_)
+    for (gh, gw) in PC.COGX_ROT_GRIDS:
+        rc, rs = pin[f"cogx_rot.grid.{gh}x{gw}"]
+        oc, os_ = CO.rotary_3d(64, CO.resize_crop_region_for_grid((gh, gw), 45, 30), (gh, gw), 5)
+        pins.assert_exact(oc, rc, (gh, gw))
+        pins.assert_exact(os_, rs, (gh, gw))
         pipe = CogVideoXPipeline.__new__(CogVideoXPipeline)
         pipe.transformer = type("T", (), {"config": type("C", (), {"patch_size": 2, "attention_head_dim": 64})()})()
         pc, ps = pipe._prepare_rotary_positional_embeddings(gh * 16, gw * 16, 5, "cpu")
-        assert torch.equal(pc, rc) and torch.equal(ps, rs)
+        pins.assert_exact(pc, rc, ("pipeline", gh, gw))
+        pins.assert_exact(ps, rs, ("pipeline", gh, gw))
     for dtype in (torch.float32, torch.bfloat16):
         x = synth.normalish("rot.x", (2, 3, 3 * 6 * 8, 64)).to(dtype)
-        c, s = _cogx_rotary()
-        assert torch.equal(E.apply_rotary_emb(x, (c, s)), CO.apply_rotary_emb(x, c, s))
+        c, s = PC.cogx_rotary()
+        pins.assert_exact(CO.apply_rotary_emb(x, c, s), pin[f"cogx_rot.apply.{PC.DT[dtype]}"], dtype)
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_cogvideox_rotary_oracle_and_mirror_vs_reference_model(monkeypatch, dtype):
+def test_cogvideox_rotary_oracle_and_mirror_vs_reference_model(pin, monkeypatch, dtype):
     """use_rotary_positional_embeddings=True (CogVideoX-5b): oracle forward (bf16 bit for bit) and, in fp32, the product front end
     on the kernel stand-ins (identity rope rows for the text tokens, RoPE-only pre-pass) against the reference model."""
     from oracle import cogvideox_oracle as CO
     from tests import kernels_emul
     from videosys_b200.models.transformers.cogvideox_transformer_3d import CogVideoXTransformer3DModel
 
-    cfg = dict(COGX_SMALL, use_rotary_positional_embeddings=True)
-    ref = ref_loader.build_cogvideox(dtype=dtype, **cfg)
-    sd = synth.fill_state_dict({k: v.float() for k, v in ref.state_dict().items()}, "cogxr.")
-    for k in sd:
-        if k.endswith("norm.weight") or k.endswith("norm_final.weight") or k.endswith("norm_q.weight") or k.endswith("norm_k.weight"):
-            sd[k] = 1.0 + 0.2 * synth.uniform("cogxr." + k, tuple(sd[k].shape))
-    sd = {k: v.to(dtype) for k, v in sd.items()}
-    ref.load_state_dict(sd)
+    cfg = dict(PC.COGX_SMALL, use_rotary_positional_embeddings=True)
+    sd = cogx_weights(pin, f"cogxr.{PC.DT[dtype]}", "cogxr.", dtype)
     lat = synth.normalish("cogxr.lat", (2, 3, 4, 12, 16)).to(dtype)
     txt = synth.normalish("cogxr.txt", (2, 16, 48)).to(dtype)
     ts = torch.tensor([499, 499])
-    rot = _cogx_rotary()
+    rot = PC.cogx_rotary()
     with torch.no_grad():
-        want = ref(lat, txt, ts, image_rotary_emb=rot, return_dict=False)[0]
-        got = CO.transformer_forward(sd, COGX_SMALL_O, lat, txt, ts, rotary=rot)
+        got = CO.transformer_forward(sd, PC.COGX_SMALL_O, lat, txt, ts, rotary=rot)
     if dtype == torch.float32:
-        assert torch.allclose(got, want, rtol=1e-4, atol=1e-5), (got - want).abs().max()
+        pins.assert_close(got, pin["cogx_rot.float32"], rtol=1e-4, atol=1e-5)
         kernels_emul.emulate(monkeypatch)
         net = CogVideoXTransformer3DModel(**cfg)
         missing, unexpected = net.load_state_dict(sd, strict=False)
         assert not missing
         out = net.eval()(lat, txt, ts, image_rotary_emb=rot, return_dict=False)[0]
-        assert torch.allclose(out, want, rtol=1e-4, atol=1e-5), (out - want).abs().max()
+        pins.assert_close(out, pin["cogx_rot.float32"], rtol=1e-4, atol=1e-5)
     else:
-        assert torch.equal(got, want)
+        pins.assert_exact(got, pin["cogx_rot.bfloat16"], "cogvideox rotary oracle bf16")

@@ -7,7 +7,7 @@ import os
 import pytest
 import torch
 
-from oracle import osp_cases as OC, synth
+from oracle import osp_cases as OC, pins, synth
 
 pytestmark = pytest.mark.gpu
 
@@ -73,6 +73,9 @@ def test_osp_v110_forward_vs_reference_golden(gold, name, dt, dn):
     out = net(x.cuda(), timestep=tt.cuda(), all_timesteps=[900, 500], encoder_hidden_states=enc.cuda(),
               attention_mask=torch.ones(x.shape[0], x.shape[2], x.shape[3], x.shape[4]), encoder_attention_mask=m,
               return_dict=False)[0].cpu()
+    if f"{name}.{dn}.rel" in gold:  # stored as a sample and the norms (oracle/pins.rel): the full outputs exceed 1 MB
+        pins.assert_rel(out, gold[f"{name}.{dn}.rel"], f"osp v110 {name} {dn}")
+        return
     r32, r16 = gold[f"{name}.fp32"], gold[f"{name}.{dn}"]
     e_ours, e_ref = _rel(out, r32), _rel(r16, r32)
     print(f"[parity] osp v110 {name} {dn}: ours-vs-reference fp32 {e_ours:.3e}, reference {dn}-vs-fp32 {e_ref:.3e}, "
